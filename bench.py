@@ -19,6 +19,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -228,6 +229,24 @@ def workload_config(rays_per_step):
                   "scratch per frame (126 MB L2)"}
 
 
+DUMP_BYTES = 64 * 10 ** 6
+
+
+def dump_outputs(out, path):
+    """Write the outputs of one step as ``path/<name>.npy`` (float32).  Above DUMP_BYTES in all, the same fixed, seeded
+    sample of rays (ascending ray order) is taken from every array, so that two builds can be compared array for array."""
+    os.makedirs(path, exist_ok=True)
+    arrays = {k: v.detach().float().cpu() for k, v in out.items()}
+    n = next(iter(arrays.values())).shape[0]
+    per_ray = sum(v[0].numel() * 4 for v in arrays.values())
+    keep = (DUMP_BYTES - 4096) // per_ray
+    if keep < n:
+        sel = torch.sort(torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep])[0]
+        arrays = {k: v[sel] for k, v in arrays.items()}
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v.numpy())
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -256,7 +275,15 @@ def main():
     ap.add_argument("--all-samples", action="store_true",
                     help="evaluate colour / nabla at every sample like the reference does, instead of only where the "
                          "visibility weight is non-zero (bit-identical outputs either way)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned (rgb, depth_volume, mask_volume, "
+                         "normals_volume) as DIR/<name>.npy, float32; a fixed sample of rays above 64 MB in all")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and (args.impl != "ours" or args.workload == "train" or args.simulate_world > 1 or args.tune):
+        ap.error("--dump-outputs writes the outputs of the timed rendering steps: not with --impl reference, "
+                 "--workload train, --simulate-world or --tune")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -378,6 +405,8 @@ def main():
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         ms_total = float(ms.item())
+        if args.dump_outputs and rank == 0:
+            dump_outputs(out, args.dump_outputs)
 
         # ---------------- same frames with every sample evaluated (reference-style work), for transparency ----------------
         g0, g1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)

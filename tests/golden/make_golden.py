@@ -20,6 +20,9 @@ ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, HERE)
 warnings.filterwarnings("ignore")
+# MKL's AVX-512 path with 8 threads, as tests/conftest.py pins it for the bit-exact comparisons
+os.environ["MKL_CBWR"] = "AVX512"
+torch.set_num_threads(8)
 
 import ref_harness  # noqa: E402
 from neumesh_b200 import synth  # noqa: E402
@@ -195,7 +198,82 @@ def make_raycast_case(name, seed):
     print("wrote", path, os.path.getsize(path), "bytes; rays hitting the surface:", int(mask.sum()), "of", mask.numel())
 
 
+def make_reference_pins(name, level, seed):
+    """What the UNMODIFIED reference computes for the CPU pins of ``tests/test_oracle.py``: its model's point queries,
+    its renderer on three small frames (no-grad; ``perturb=True`` under grad with ``samples_output``; ``perturb=True``
+    with the uniforms handed to it through a patched ``torch.rand``) and ``rend_util.sample_pdf``."""
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import helpers
+    ns = ref_harness.load()
+    cfg = synth.ModelConfig()
+    mesh = synth.icosphere_mesh(level, seed=seed)
+    sd = synth.make_state_dict(mesh, cfg, seed=seed + 1)
+    ref = ref_harness.build_reference_model(mesh, cfg, sd)
+    # inputs, stored with the outputs: point queries, three small frames, sample_pdf bins / weights, perturb uniforms
+    x, v = helpers.sample_points(500, seed=1)
+    torch.manual_seed(0)
+    bins = torch.sort(torch.rand(64, 40), dim=-1)[0]
+    wts = torch.rand(64, 39) * (torch.rand(64, 39) > 0.5)
+    inp = dict(xyz=x, view_dirs=v, pdf_bins=bins, pdf_weights=wts)
+    for tag, n, view in (("render", 10, 1), ("dropin", 8, 2), ("perturb", 9, 4)):
+        inp[tag + "_rays_o"], inp[tag + "_rays_d"] = synth.frame_rays(n, n, view=view)
+    inp["perturb_u"] = torch.rand(4, n * n, 16, generator=torch.Generator().manual_seed(11))
+    out = dict(level=np.int64(level), seed=np.int64(seed), state_digest=np.array(state_digest(sd)))
+    out.update({k: t.numpy() for k, t in inp.items()})
+    with torch.no_grad():
+        out["sdf"] = ref.forward_density_only(x).numpy()
+    s, n = ref.forward_with_nablas(x.clone())
+    out["sdf_with_nabla"], out["nabla"] = s.detach().numpy(), n.detach().numpy()
+    _, c = ref.forward(x.clone(), v)
+    out["rgb_pts"] = c.detach().numpy()
+    kw = dict(calc_normal=True, white_bkgd=True, bounded_near_far=True, detailed_output=True, rayschunk=64)
+    with torch.no_grad():
+        _, _, ex = ns.renderer.volume_render(inp["render_rays_o"], inp["render_rays_d"], ref, **kw)
+    for k in ("rgb", "depth_volume", "mask_volume", "normals_volume", "d_final", "implicit_surface", "radiance"):
+        out["render_" + k] = ex[k].numpy()
+    out["pdf_samples"] = ns.rend_util.sample_pdf(inp["pdf_bins"], inp["pdf_weights"], 16, det=True).numpy()
+    # the keys the reference renderer returns: the drop-in renderer must return at least these
+    o, d = inp["dropin_rays_o"], inp["dropin_rays_d"]
+    with torch.no_grad():
+        rgb, dep, ex = ns.renderer.volume_render(o, d, ref, **kw)
+    out.update(dropin_rgb=rgb.numpy(), dropin_depth=dep.numpy(), dropin_keys=np.array(sorted(ex)))
+    # a training-style call: grad enabled, perturb=True (draws from torch's CPU generator), samples_output
+    ref.train()
+    torch.manual_seed(3)
+    rgb, dep, ex = ns.renderer.volume_render(o, d, ref, calc_normal=True, detailed_output=True, samples_output=True,
+                                             perturb=True, rayschunk=64)
+    ref.eval()
+    out.update(train_rgb=rgb.detach().numpy(), train_depth=dep.detach().numpy(), train_keys=np.array(sorted(ex)))
+    # perturb=True with the uniforms injected: torch.rand is patched to hand out perturb_u, one [N, 16] slab per call
+    u = inp["perturb_u"]
+    calls = {"n": 0}
+    real_rand = torch.rand
+
+    def fake_rand(*shape, **kw):
+        shp = tuple(shape[0]) if len(shape) == 1 and isinstance(shape[0], (list, tuple)) else tuple(shape)
+        r = u[calls["n"]].reshape(shp).clone()
+        calls["n"] += 1
+        return r
+
+    torch.rand = fake_rand
+    try:
+        with torch.no_grad():
+            rgb, dep, ex = ns.renderer.volume_render(inp["perturb_rays_o"], inp["perturb_rays_d"], ref,
+                                                     detailed_output=True, perturb=True, rayschunk=4096,
+                                                     calc_normal=True, white_bkgd=False, bounded_near_far=True)
+    finally:
+        torch.rand = real_rand
+    out.update(perturb_rgb=rgb.numpy(), perturb_depth=dep.numpy(), perturb_d_final=ex["d_final"].numpy(),
+               perturb_rand_calls=np.int64(calls["n"]))
+    path = os.path.join(HERE, name + ".npz")
+    np.savez_compressed(path, **out)
+    print("wrote", path, os.path.getsize(path), "bytes")
+
+
 def main():
+    if len(sys.argv) > 1 and sys.argv[1] == "pins":
+        make_reference_pins("reference_pins_small", 3, seed=5)
+        return
     if len(sys.argv) > 1 and sys.argv[1] == "raycast":
         make_raycast_case("ray_casting_small", seed=60)
         return
@@ -218,6 +296,7 @@ def main():
     make_texture_case("texture_edit_small", seed=40)
     make_neus_case("neus_teacher_small", seed=50)
     make_raycast_case("ray_casting_small", seed=60)
+    make_reference_pins("reference_pins_small", 3, seed=5)
 
 
 if __name__ == "__main__":

@@ -1,5 +1,6 @@
-"""CPU tests: the oracle is pinned (a) against the committed golden vectors that the UNMODIFIED reference produced
-and (b), when the reference tree is present (build container), against the reference itself, bit for bit."""
+"""CPU tests: the oracle (and, on CPU, the drop-in model and renderer) is pinned against the committed golden vectors
+that the UNMODIFIED reference produced (``tests/golden/make_golden.py``), bit for bit where the same torch ops run in
+the same order."""
 import os
 
 import numpy as np
@@ -60,111 +61,77 @@ def test_knn_oracle_brute_vs_kdtree():
     assert torch.allclose(dists[0, :, 0], ((q - p[idxs[0, :, 0]]) ** 2).sum(-1), atol=1e-7)
 
 
-def test_oracle_vs_unmodified_reference():
-    """Only where /root/reference exists (the build container)."""
-    import ref_harness
-    if not ref_harness.available():
-        pytest.skip("reference tree not present (GPU box)")
-    ns = ref_harness.load()
-    cfg = synth.ModelConfig()
-    mesh = synth.icosphere_mesh(3, seed=5)
-    sd = synth.make_state_dict(mesh, cfg, seed=6)
-    ref = ref_harness.build_reference_model(mesh, cfg, sd)
+def _pins(golden_dir):
+    g, mesh, cfg, sd, _ = helpers.golden_case(os.path.join(golden_dir, "reference_pins_small.npz"))
+    t = {k: torch.from_numpy(v) for k, v in g.items() if v.dtype == np.float32}
+    return g, t, mesh, cfg, sd
+
+
+def test_oracle_vs_unmodified_reference(golden_dir):
+    """The oracle's field, renderer and inverse-CDF sampler equal, bit for bit, what the unmodified reference computed
+    for the same inputs (``tests/golden/make_golden.py pins``)."""
+    g, t, mesh, cfg, sd = _pins(golden_dir)
     f = helpers.oracle_field(mesh, cfg, sd)
-    x, v = helpers.sample_points(500, seed=1)
-    with torch.no_grad():
-        assert torch.equal(ref.forward_density_only(x), f.forward_density_only(x))
-    s_r, n_r = ref.forward_with_nablas(x.clone())
+    x, v = t["xyz"], t["view_dirs"]
+    assert torch.equal(t["sdf"], f.forward_density_only(x))
     s_o, n_o = f.forward_with_nablas(x)
-    assert torch.equal(n_r, n_o) and torch.equal(s_r.detach(), s_o)
-    _, c_r = ref.forward(x.clone(), v)
+    assert torch.equal(t["nabla"], n_o) and torch.equal(t["sdf_with_nabla"], s_o)
     _, c_o = f.forward(x, v)
-    assert torch.equal(c_r.detach(), c_o)
-    o, d = synth.frame_rays(10, 10, view=1)
+    assert torch.equal(t["rgb_pts"], c_o)
     kw = dict(calc_normal=True, white_bkgd=True, bounded_near_far=True)
-    with torch.no_grad():
-        rgb_r, dep_r, ex_r = ns.renderer.volume_render(o, d, ref, detailed_output=True, rayschunk=64, **kw)
-    rgb_o, dep_o, ex_o = orender.volume_render(o, d, f, detailed_output=True, rayschunk=64, **kw)
+    rgb_o, dep_o, ex_o = orender.volume_render(t["render_rays_o"], t["render_rays_d"], f, detailed_output=True,
+                                               rayschunk=64, **kw)
     for k in ("rgb", "depth_volume", "mask_volume", "normals_volume", "d_final", "implicit_surface", "radiance"):
-        assert torch.equal(ex_r[k], ex_o[k]), k
+        assert torch.equal(t["render_" + k], ex_o[k]), k
     # sample_pdf on its own, incl. the u = 0 / u = 1 ends (SURVEY.md section 8a')
-    torch.manual_seed(0)
-    bins = torch.sort(torch.rand(64, 40), dim=-1)[0]
-    wts = torch.rand(64, 39) * (torch.rand(64, 39) > 0.5)
-    assert torch.equal(ns.rend_util.sample_pdf(bins, wts, 16, det=True), orender.inverse_cdf_samples(bins, wts, 16))
+    assert torch.equal(t["pdf_samples"], orender.inverse_cdf_samples(t["pdf_bins"], t["pdf_weights"], 16))
 
 
-def test_reference_renderer_and_trainer_loss_run_on_the_dropin_model():
-    """INTEGRATION.md section 3 end to end, as far as a CPU allows: the UNMODIFIED ``models/renderer.py::volume_render``
-    drives the drop-in ``neumesh_b200.NeuMesh`` (its protocol is all the reference's renderer touches), no-grad and under
-    autograd with ``perturb=True``, and the result equals what the reference renders with its own model."""
-    import ref_harness
-    if not ref_harness.available():
-        pytest.skip("reference tree not present (GPU box)")
+def test_reference_renderer_and_trainer_loss_run_on_the_dropin_model(golden_dir):
+    """INTEGRATION.md section 3 end to end, as far as a CPU allows: the drop-in ``neumesh_b200.NeuMesh`` loads the
+    reference's state_dict and, driven by the drop-in renderer and by the oracle's restatement of the reference renderer
+    (``models/renderer.py::volume_render``), renders what the reference renders with its own model; under autograd with
+    ``perturb=True`` it returns every key the reference's renderer returns to the trainer, and its loss back-propagates."""
     import neumesh_b200 as nb
-    ns = ref_harness.load()
-    cfg = synth.ModelConfig()
-    mesh = synth.icosphere_mesh(3, seed=5)
-    sd = synth.make_state_dict(mesh, cfg, seed=6)
-    ref = ref_harness.build_reference_model(mesh, cfg, sd)
+    g, t, mesh, cfg, sd = _pins(golden_dir)
     ours = nb.NeuMesh(helpers.OracleMeshGrid(mesh), **cfg.model_kwargs())
     ours.load_state_dict(sd, strict=True)      # identical state_dict keys
     ours.eval()
-    o, d = synth.frame_rays(8, 8, view=2)
+    o, d = t["dropin_rays_o"], t["dropin_rays_d"]
+    rgb_r, dep_r = t["dropin_rgb"], t["dropin_depth"]
     kw = dict(calc_normal=True, white_bkgd=True, bounded_near_far=True, detailed_output=True, rayschunk=64)
     with torch.no_grad():
-        rgb_r, dep_r, ex_r = ns.renderer.volume_render(o, d, ref, **kw)
-        rgb_o, dep_o, ex_o = ns.renderer.volume_render(o, d, ours, **kw)          # reference renderer, drop-in model
+        rgb_o, dep_o, _ = orender.volume_render(o, d, ours, **kw)                 # reference renderer (restated), drop-in model
         rgb_n, dep_n, ex_n = nb.volume_render(o, d, ours, **kw)                   # drop-in renderer, drop-in model
-    assert set(ex_r.keys()) == set(ex_o.keys()) <= set(ex_n.keys()) | {"near_far"}
+    assert set(g["dropin_keys"]) <= set(ex_n.keys()) | {"near_far"}
     for a, b in ((rgb_o, rgb_r), (dep_o, dep_r), (rgb_n, rgb_r), (dep_n, dep_r)):
         assert (a - b).abs().max() < 1e-5
     # training-style call: grad enabled, perturb=True (the reference's default), samples_output for the distillation loss
     ours.train()
     ours.fused_train = False
     torch.manual_seed(3)
-    rgb_t, dep_t, ex_t = ns.renderer.volume_render(o, d, ours, calc_normal=True, detailed_output=True, samples_output=True,
-                                                   perturb=True, rayschunk=64)
-    assert {"xyz", "dirs", "density", "colors", "implicit_nablas"} <= set(ex_t.keys())
+    rgb_t, dep_t, ex_t = nb.volume_render(o, d, ours, calc_normal=True, detailed_output=True, samples_output=True,
+                                          perturb=True, rayschunk=64)
+    assert {"xyz", "dirs", "density", "colors", "implicit_nablas"} <= set(g["train_keys"]) <= set(ex_t.keys())
+    assert (rgb_t - t["train_rgb"]).abs().max() < 1e-5 and (dep_t - t["train_depth"]).abs().max() < 1e-5
     loss = helpers.train_loss(rgb_t, dep_t, ex_t) + ex_t["density"].abs().mean() + ex_t["colors"].mean()
     loss.backward()
     assert all(p.grad is not None and torch.isfinite(p.grad).all() for n, p in ours.named_parameters()
                if n != "indicator_weight_raw")
 
 
-def test_oracle_perturb_with_injected_uniforms_equals_reference_with_patched_rand():
+def test_oracle_perturb_with_injected_uniforms_equals_reference_with_patched_rand(golden_dir):
     """perturb=True (rend_util.py:292-295) draws ``torch.rand`` once per up-sampling iteration; the oracle takes the draws
-    as ``perturb_u``.  With ``torch.rand`` patched to hand the reference the same draws, both renders are bit-identical."""
-    import ref_harness
-    if not ref_harness.available():
-        pytest.skip("reference tree not present (GPU box)")
-    ns = ref_harness.load()
-    cfg = synth.ModelConfig()
-    mesh = synth.icosphere_mesh(3, seed=5)
-    sd = synth.make_state_dict(mesh, cfg, seed=6)
-    ref = ref_harness.build_reference_model(mesh, cfg, sd)
+    as ``perturb_u``.  The reference, with ``torch.rand`` patched to hand it the same draws, drew them four times and
+    rendered what the oracle renders, bit for bit."""
+    g, t, mesh, cfg, sd = _pins(golden_dir)
     f = helpers.oracle_field(mesh, cfg, sd)
-    o, d = synth.frame_rays(9, 9, view=4)
-    u = torch.rand(4, o.shape[0], 16, generator=torch.Generator().manual_seed(11))
-    calls = {"n": 0}
-    real_rand = torch.rand
-
-    def fake_rand(*shape, **kw):
-        shp = tuple(shape[0]) if len(shape) == 1 and isinstance(shape[0], (list, tuple)) else tuple(shape)
-        out = u[calls["n"]].reshape(shp).clone()
-        calls["n"] += 1
-        return out
-
+    o, d, u = t["perturb_rays_o"], t["perturb_rays_d"], t["perturb_u"]
+    assert int(g["perturb_rand_calls"]) == u.shape[0] == 4
     kw = dict(calc_normal=True, white_bkgd=False, bounded_near_far=True)
-    torch.rand = fake_rand
-    try:
-        with torch.no_grad():
-            rgb_r, dep_r, ex_r = ns.renderer.volume_render(o, d, ref, detailed_output=True, perturb=True, rayschunk=4096, **kw)
-    finally:
-        torch.rand = real_rand
-    assert calls["n"] == 4
     rgb_o, dep_o, ex_o = orender.volume_render(o, d, f, detailed_output=True, perturb_u=u, **kw)
-    assert torch.equal(rgb_r, rgb_o) and torch.equal(dep_r, dep_o) and torch.equal(ex_r["d_final"], ex_o["d_final"])
+    assert torch.equal(t["perturb_rgb"], rgb_o) and torch.equal(t["perturb_depth"], dep_o)
+    assert torch.equal(t["perturb_d_final"], ex_o["d_final"])
     # and it differs from the deterministic render (the draws are used)
     rgb_d, _, _ = orender.volume_render(o, d, f, **kw)
     assert not torch.equal(rgb_d, rgb_o)
