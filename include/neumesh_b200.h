@@ -204,6 +204,24 @@ int nmb_pack_bgr8(const float* rgb, int64_t N, uint8_t* bgr8, void* stream);
 int nmb_vertex_normals(const float* vertices, int64_t V, const int32_t* triangles, int64_t T, float* normals,
                        void* stream);
 
+/* ---- mesh extraction -----------------------------------------------------------------------------------------
+ * Marching cubes (mcubes.marching_cubes(volume, iso) at extract_mesh.py:138) on a dense fp32 volume [n0,n1,n2]
+ * (C order, every dim >= 2, at most 2^34 points).  Output in index space: vertices [Nv,3] float64 along axes
+ * (0, 1, 2), triangles [Nt,3] int64.  Conventions (csrc/mcubes.cu, DESIGN.md section 4.8): a point is inside iff
+ * value < iso; one vertex per crossing grid edge, owned by the edge's lower end p, at p + t e_a with
+ * t = (iso - v(p)) / (v(p + e_a) - v(p)) in float64 without contraction; vertices ordered by (owner's linear index,
+ * axis), triangles by (cell linear index, position in the case table); the right-hand normal of every triangle points
+ * toward values >= iso.  Tables: csrc/mc_tables.cuh.
+ * Usage: workspace of nmb_mc_workspace_bytes() bytes (-1: dimensions rejected, see nmb_last_error); nmb_mc_count
+ * classifies and scans, then SYNCHRONISES the stream to return the totals to the host; nmb_mc_emit (same volume, iso
+ * and workspace, nothing in between) writes vertices and triangles (either may be NULL).  An empty surface gives
+ * zero counts. */
+int64_t nmb_mc_workspace_bytes(int64_t n0, int64_t n1, int64_t n2);
+int nmb_mc_count(const float* vol, int64_t n0, int64_t n1, int64_t n2, double iso, void* workspace,
+                 int64_t workspace_bytes, int64_t* n_vertices /*HOST*/, int64_t* n_triangles /*HOST*/, void* stream);
+int nmb_mc_emit(const float* vol, int64_t n0, int64_t n1, int64_t n2, double iso, void* workspace,
+                int64_t workspace_bytes, double* vertices, int64_t* triangles, void* stream);
+
 /* ---- training-path primitives (config 4: forward + backward through the field) -----------------------------------
  * The reference trains through the renderer with autograd: models/trainer.py:75-80 (forward), :173-262 (losses on rgb,
  * mask_volume, implicit_nablas, density, colors), neumesh.py:204-260 (field; the nabla comes from
@@ -212,7 +230,8 @@ int nmb_vertex_normals(const float* vertices, int64_t V, const int32_t* triangle
  * dense row-major fp32 in the caller's layouts (torch parameter tensors, ORIGINAL vertex order, weights [out, in]).
  * Derivation of the backward formulas and a float64 check against autograd: tools/train_math_proto.py. */
 
-/* C[M,N] (+)= A.B (+ bias[N]) with epilogue 0 none | 1 relu | 2 zero where mask[m*ldmask + n] <= 0.
+/* C[M,N] (+)= A.B (+ bias[N]) with epilogue 0 none | 1 relu | 2 zero where mask[m*ldmask + n] <= 0 |
+ * 3 softplus(beta = 100, threshold = 20) (the NeuS teacher's hidden layers, value rows only).
  * A(m,k) = a_kcontig ? A[m*lda + k] : A[k*lda + m];  B(k,n) = b_kcontig ? B[n*ldb + k] : B[k*ldb + n].
  * (torch.nn.Linear forward: a_kcontig = b_kcontig = 1; dX = dZ.W: (1, 0); dW = dZ^T.X: (0, 0), split over K.) */
 int nmb_tr_gemm(const float* A, int64_t lda, int a_kcontig, const float* B, int64_t ldb, int b_kcontig, float* C,

@@ -74,6 +74,9 @@ SIGNATURES = {
     "nmb_pack_bgr8": (C.c_int, [_P, _I64, _P, _P]),
     "nmb_vertex_normals": (C.c_int, [_P, _I64, _P, _I64, _P, _P]),
     "nmb_get_rays": (C.c_int, [C.POINTER(_F), C.POINTER(_F), _I32, _I32, _P, _P, _P]),
+    "nmb_mc_workspace_bytes": (_I64, [_I64, _I64, _I64]),
+    "nmb_mc_count": (C.c_int, [_P, _I64, _I64, _I64, C.c_double, _P, _I64, C.POINTER(_I64), C.POINTER(_I64), _P]),
+    "nmb_mc_emit": (C.c_int, [_P, _I64, _I64, _I64, C.c_double, _P, _I64, _P, _P, _P]),
     # training-path primitives (csrc/train.cu); the nmb_tr_inputs struct is bound in train_ops.TrInputs
     "nmb_tr_gemm": (C.c_int, [_P, _I64, C.c_int, _P, _I64, C.c_int, _P, _I64, _I64, _I64, _I64, _P, C.c_int, _P, _I64,
                               C.c_int, _P]),

@@ -13,7 +13,8 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_DIR = os.path.join(HERE, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libneumesh_b200.so")
-SOURCES = ["api.cu", "grid.cu", "field.cu", "field_ffma.cu", "field_tc.cu", "render.cu", "shell.cu", "train.cu"]
+SOURCES = ["api.cu", "grid.cu", "field.cu", "field_ffma.cu", "field_tc.cu", "render.cu", "shell.cu", "train.cu",
+           "mcubes.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC",
               "--expt-relaxed-constexpr"]
 

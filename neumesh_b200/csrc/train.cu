@@ -36,6 +36,13 @@ namespace tr {
 // ------------------------------------------------------------------------------------------------------------
 constexpr int BM = 128, BN = 128, BK = 16, PAD = 4;
 
+__device__ __forceinline__ void softplus_terms(float z, float& sp, float& s1, float& s2);
+__device__ __forceinline__ float softplus100(float z) {
+  float sp, s1, s2;
+  softplus_terms(z, sp, s1, s2);
+  return sp;
+}
+
 template <bool A_KC, bool B_KC>
 __global__ void __launch_bounds__(256, 2)
 sgemm_kernel(int M, int N, int K, const float* __restrict__ A, int64_t lda, const float* __restrict__ B, int64_t ldb,
@@ -117,6 +124,7 @@ sgemm_kernel(int M, int N, int K, const float* __restrict__ A, int64_t lda, cons
       if (bias) v += bias[gn];
       if (epi == 1) v = fmaxf(v, 0.f);
       if (epi == 2) v = (mask[(int64_t)gm * ldmask + gn] > 0.f) ? v : 0.f;
+      if (epi == 3) v = softplus100(v);
       float* dst = Cz + (int64_t)gm * ldc + gn;
       if (accumulate) v += *dst;
       *dst = v;
@@ -555,7 +563,7 @@ int nmb_tr_gemm(const float* A, int64_t lda, int a_kcontig, const float* B, int6
   using namespace nmb::tr;
   NMB_CHECK(A && B && C, "null argument");
   NMB_CHECK(M < (int64_t(1) << 31) && N < (int64_t(1) << 31) && K < (int64_t(1) << 31), "dimension too large");
-  NMB_CHECK(epilogue >= 0 && epilogue <= 2 && (epilogue != 2 || mask), "bad epilogue");
+  NMB_CHECK(epilogue >= 0 && epilogue <= 3 && (epilogue != 2 || mask), "bad epilogue");
   if (M <= 0 || N <= 0) return 0;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   const int gm = (int)ceil_div(M, BM), gn = (int)ceil_div(N, BN);

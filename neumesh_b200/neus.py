@@ -247,6 +247,39 @@ def _fused_surface(surf: ImplicitSurface, x):
     return sdf.reshape(lead), nabla.reshape(*lead, 3), feat.reshape(*lead, N - 1)
 
 
+def _fused_surface_value(surf: ImplicitSurface, x):
+    """-> sdf [M] of flat points x [M,3]: the value row block of ``_fused_surface`` alone (no tangent rows, no feature
+    columns), for dense grids where only the sdf is kept.  Each hidden layer is one ``nmb_tr_gemm`` with the bias +
+    softplus(beta = 100) epilogue, which computes the same fp32 operations as ``_fused_surface``'s value rows, so the
+    two agree bit for bit; every row is independent, so the result does not depend on how the caller chunks x."""
+    from . import train_ops
+    flat = x.detach().reshape(-1, 3).float().contiguous()
+    M, dev = flat.shape[0], flat.device
+    P = train_ops.CudaPrims(dev)
+    cols = [flat]
+    for k in range(max(surf.embed_multires, 0)):        # the value columns of _embed_with_jacobian, same operations
+        f = 2.0 ** k
+        cols += [torch.sin(flat * f), torch.cos(flat * f)]
+    X0 = torch.cat(cols, -1).contiguous()
+    H = X0
+    inv_sqrt2 = 1.0 / np.sqrt(2)
+    for i in range(surf.D):
+        if i in surf.skips:
+            H = (torch.cat([H, X0], dim=-1) * inv_sqrt2).contiguous()
+        lin = surf.surface_fc_layers[i]
+        Wt = _eff_weight(lin).detach().float().contiguous()
+        N, K = Wt.shape
+        Z = torch.empty(M, N, device=dev)
+        P.gemm(H, H.shape[1], True, Wt, K, True, Z, N, M, N, K, bias=lin.bias.detach().float().contiguous(), epilogue=3)
+        H = Z
+    lin = surf.surface_fc_layers[-1]
+    Wt = _eff_weight(lin).detach().float()[:1].contiguous()     # row 0 is the sdf; the rest is the geometry feature
+    K = Wt.shape[1]
+    sdf = torch.empty(M, 1, device=dev)
+    P.gemm(H, H.shape[1], True, Wt, K, True, sdf, 1, M, 1, K, bias=lin.bias.detach().float()[:1].contiguous())
+    return sdf.reshape(M)
+
+
 def _fused_radiance(net: RadianceNet, inp):
     from . import train_ops
     lead = inp.shape[:-1]
